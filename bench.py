@@ -10,6 +10,10 @@ step   : one pass of the hot path over the whole 4000-step sequence.
 
     python bench.py --gpus N --steps K --warmup W          # this repo
     python bench.py --impl reference ...                   # CPU arm (oracle port)
+    python bench.py ... --dump-outputs DIR                 # + what the last timed step computed, as DIR/*.npy
+
+The run writes nothing into the repository tree: it loads libpulser_b200.so as
+build() left it and keeps Python from caching bytecode next to the sources.
 
 N > 1: one process per GPU (torchrun).  `value` stays C2: the single-state path
 does not shard ("replicas only", DESIGN.md), every GPU evolves the same Sequence,
@@ -39,11 +43,13 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True
 
 N_ATOMS = int(os.environ.get("PB200_BENCH_ATOMS", "20"))
 INTEGRATOR_NAMES = {1: "chebyshev-clenshaw (Richardson-CF4 Magnus)", 2: "lanczos (Richardson-CF4 Magnus)", 3: "time-dependent taylor"}
 METRIC = "time-steps/s (1 ns sampling intervals of the Sequence evolved per second)"
 UNIT = "steps/s"
+DUMP_BYTES = 48 << 20   # at most this much of the final state in --dump-outputs (a seeded sample above it)
 
 
 def workload(seed: int):
@@ -365,11 +371,23 @@ def c5_leg(local: int, stream, peak: float) -> dict:
 
 
 # --------------------------------------------------------------------------
+def dump_outputs(out_dir: str, psi: np.ndarray, dens: np.ndarray) -> None:
+    """What the last timed step computed: the final C2 state as float64 (re, im) pairs (c2_state.npy, [D, 2]) and the
+    per-atom Rydberg densities derived from it (c2_rydberg_density.npy).  Above DUMP_BYTES the state is a fixed,
+    seeded sample of amplitudes, whose indices go to c2_state_index.npy (float64, exact below 2^53)."""
+    os.makedirs(out_dir, exist_ok=True)
+    state = np.ascontiguousarray(psi).view(np.float64).reshape(-1, 2)
+    if state.nbytes > DUMP_BYTES:
+        idx = np.sort(np.random.default_rng(0).choice(len(state), size=DUMP_BYTES // 16, replace=False))
+        state = state[idx]
+        np.save(os.path.join(out_dir, "c2_state_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, "c2_state.npy"), state)
+    np.save(os.path.join(out_dir, "c2_rydberg_density.npy"), np.asarray(dens, dtype=np.float64))
+
+
 def run_gpu(args) -> None:
     import torch
 
-    from pulser_b200 import build
-    build.build()
     from pulser_b200 import engine
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -419,6 +437,7 @@ def run_gpu(args) -> None:
             barrier()
             times_ms.append(e0.elapsed_time(e1))
             launches += st["n_launches"]; applies += st["n_applies"]; kernel_ms += st["gpu_ms"]
+    psi_final = plan.get_state()[0] if args.dump_outputs and rank == 0 else None
     norm2 = float(plan.norm2()[0])
     # final observable of this replica: Rydberg density per atom (host side, from |psi|^2)
     probs = plan.probabilities()[0]
@@ -432,6 +451,8 @@ def run_gpu(args) -> None:
         dist.all_reduce(obs, op=dist.ReduceOp.SUM)    # THE collective of the path: final expectation values
     total_ms = float(t_all.item())
     value = world * T * args.steps / (total_ms * 1e-3)
+    if psi_final is not None:
+        dump_outputs(args.dump_outputs, psi_final, dens)
 
     # ---- end to end through the public API with host buffers ----
     psi0_host = np.zeros(D, dtype=np.complex128)
@@ -513,12 +534,23 @@ def run_gpu(args) -> None:
         dist.destroy_process_group()
 
 
+def _count(minimum: int):
+    def parse(text: str) -> int:
+        v = int(text)
+        if v < minimum:
+            raise argparse.ArgumentTypeError(f"must be >= {minimum}, got {v}")
+        return v
+    return parse
+
+
 def main() -> None:
     ap = argparse.ArgumentParser()
-    ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--gpus", type=_count(1), default=1)
+    ap.add_argument("--steps", type=_count(1), default=5, help="timed steps (passes over the whole sequence)")
+    ap.add_argument("--warmup", type=_count(0), default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/*.npy (b200 arm)")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

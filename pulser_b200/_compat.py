@@ -8,8 +8,7 @@ Its only hard non-numeric dependency is matplotlib (drawing only,
 meta-path finder serves empty stand-in modules for ``matplotlib.*``.
 
 pulser is OPTIONAL: the CUDA path, the C-ABI and the plain-array
-``HamiltonianSpec`` entry point work without it (the GPU box has no
-``/root/reference``).
+``HamiltonianSpec`` entry point work without it.
 """
 from __future__ import annotations
 
@@ -20,10 +19,8 @@ import os
 import sys
 import types
 
-_REFERENCE_CORE = "/root/reference/pulser-core"
-# offline install of the unmodified pulser-core (python -m pip install --no-deps --target baseline/_ref
-# /root/reference/pulser-core, DESIGN.md section 5): git-ignored, travels to the GPU box with the repository snapshot
-_INSTALLED_CORE = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "baseline", "_ref")
+# copy of the unmodified pulser-core that build() makes with oracle/ref_build.py (git-ignored, DESIGN.md section 5)
+_BUILT_CORE = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref", "pulser-core")
 
 
 class _Anything:
@@ -90,7 +87,7 @@ def ensure_pulser() -> bool:
         if not any(isinstance(f, _DrawingStubFinder) for f in sys.meta_path):
             sys.meta_path.append(_DrawingStubFinder())
     if not _have("pulser"):
-        for root in (os.environ.get("PULSER_B200_PULSER_PATH"), _REFERENCE_CORE, _INSTALLED_CORE):
+        for root in (os.environ.get("PULSER_B200_PULSER_PATH"), _BUILT_CORE):
             if root and os.path.isdir(os.path.join(root, "pulser")):
                 sys.path.insert(0, root)
                 break

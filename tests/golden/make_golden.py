@@ -1,15 +1,18 @@
-"""Generate the committed golden fixtures from the REAL reference (pulser-core
-imported from /root/reference) plus the tight-tolerance oracle.
+"""Generate the committed golden fixtures from the REAL reference (pulser-core,
+imported from the copy that __graft_entry__.build() makes under oracle/_ref)
+plus the tight-tolerance oracle.
 
-Run in the build container only (the GPU box has no /root/reference):
-    python tests/golden/make_golden.py [--extra | --xy | --slm | --counters]
+Run where pulser-core is importable:
+    python tests/golden/make_golden.py [--extra | --xy | --slm | --counters | --workloads]
 
 Each ``*.npz`` holds a HamiltonianSpec (what the reference's Hamiltonian
 constructor receives, extracted from real pulser objects), an initial state and
 the expected output.  Sources of the expected values:
   * ``ref_*``  : numbers hard-coded in the reference's own tests
                  (tests/pulser_simulation/test_simulation.py etc., cited below);
-  * ``orc_*``  : oracle (oracle/evolve.py, DOP853 rtol 1e-13) on the same spec.
+  * ``orc_*``  : oracle (oracle/evolve.py, DOP853 rtol 1e-13) on the same spec;
+  * ``pul_*``  : what pulser-core itself computes (drive tables, interaction
+                 matrices) for the Sequences that pulser_b200/workloads.py restates.
 """
 import os
 import sys
@@ -164,7 +167,7 @@ def main():
         save(f"orc_noisy_traj{i}", spec, psi0=psi0, orc_final=oracle_final(spec, psi0), reps=reps)
 
 
-if __name__ == "__main__" and "--extra" not in sys.argv and "--xy" not in sys.argv and "--slm" not in sys.argv and "--counters" not in sys.argv:
+if __name__ == "__main__" and not {"--extra", "--xy", "--slm", "--counters", "--workloads"} & set(sys.argv):
     main()
 
 
@@ -563,3 +566,81 @@ if __name__ == "__main__" and "--counters" in sys.argv:
     if "--expect-only" not in sys.argv:
         eom_counters()
     expect_leakage()
+
+
+def workloads():
+    """pul_workloads.npz: what pulser-core computes for the Sequences that pulser_b200/workloads.py restates as plain
+    arrays (tests/test_oracle_cpu.py compares the restatements with it).  Drive tables are stored as a seeded sample
+    of their columns plus a digest of all of them (tests/helpers.py::table_sample), the rest in full."""
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    from helpers import table_sample
+    from pulser.devices import AnalogDevice
+    from pulser_b200 import workloads as W
+
+    out = {}
+
+    def put(case, spec, tables=True):
+        out[f"{case}_eigenbasis"] = np.array(spec.eigenbasis)
+        out[f"{case}_basis_name"] = np.array(spec.basis_name)
+        out[f"{case}_interaction_type"] = np.array(spec.interaction_type)
+        out[f"{case}_interaction_matrix"] = spec.interaction_matrix
+        out[f"{case}_sampling_times"] = spec.sampling_times
+        out[f"{case}_drive_bases"] = np.array([d.basis for d in spec.drives])
+        for i, d in enumerate(spec.drives):
+            if tables:
+                out[f"{case}_d{i}_coef_cols"], out[f"{case}_d{i}_coef_digest"] = table_sample(d.coef)
+                out[f"{case}_d{i}_det_cols"], out[f"{case}_d{i}_det_digest"] = table_sample(d.det)
+            else:
+                out[f"{case}_d{i}_coef"], out[f"{case}_d{i}_det"] = d.coef, d.det
+
+    om = 2 * np.pi * 1.5
+    U = om / 2
+
+    def sweep(seq):
+        seq.declare_channel("ch", "rydberg_global")
+        seq.add(Pulse.ConstantDetuning(RampWaveform(500, 0, om), -6 * U, 0), "ch")
+        seq.add(Pulse.ConstantAmplitude(om, RampWaveform(2500, -6 * U, 2 * U), 0), "ch")
+        seq.add(Pulse.ConstantDetuning(RampWaveform(1000, om, 0), 2 * U, 0), "ch")
+        return seq
+
+    # C1: 2 x 2 square, one constant pi pulse
+    seq = Sequence(Register.square(2, spacing=6.0, prefix="q"), MockDevice)
+    seq.declare_channel("ch", "rydberg_global")
+    seq.add(Pulse.ConstantPulse(1000, 2 * np.pi, np.pi, 0), "ch")
+    put("c1", specs_of(seq)[0][0])
+    # C2 at 9 atoms: the blockade sweep on the random disc register
+    n = 9
+    coords = W.disc_register(n, 38.0, 5.0, n)
+    put("c2", specs_of(sweep(Sequence(Register.from_coordinates(coords, center=False, prefix="q"), AnalogDevice)))[0][0])
+    # C3 at 5 atoms: raman pi/2 - rydberg pi - raman pi/2 in the 'all' basis
+    n = 5
+    coords = W.disc_register(n, 22.0, 6.0, 100 + n)
+    seq = Sequence(Register.from_coordinates(coords, center=False, prefix="q"), MockDevice)
+    seq.declare_channel("ram", "raman_global")
+    seq.declare_channel("ryd", "rydberg_global")
+    seq.add(Pulse.ConstantDetuning(BlackmanWaveform(500, np.pi / 2), 0, 0), "ram")
+    seq.add(Pulse.ConstantDetuning(BlackmanWaveform(1000, np.pi), 0, 0), "ryd", protocol="wait-for-all")
+    seq.add(Pulse.ConstantDetuning(BlackmanWaveform(500, np.pi / 2), 0, 0), "ram", protocol="wait-for-all")
+    put("c3", specs_of(seq)[0][0])
+    # C4: two doppler + amplitude noise trajectories of the 4 x 4 sweep, with the noise they drew
+    seq = sweep(Sequence(Register.square(4, spacing=6.0, prefix="q"), MockDevice))
+    np.random.seed(3)
+    hd, T = hdata(seq, NoiseModel(temperature=50.0, amp_sigma=0.05, laser_waist=175.0), 2)
+    for i, (tr, ns, _) in enumerate(hd.noisy_samples):
+        put(f"c4_{i}", spec_from_pulser(ns, tr, hd.basis_data, hd.lindblad_data, 1.0, T))
+        out[f"c4_{i}_doppler"] = np.array([tr.doppler_detune[q] for q in seq.register.qubit_ids])
+        out[f"c4_{i}_amp"] = np.array(tr.amp_fluctuations["ch"])
+    # XY: a global microwave pulse under a tilted field, 5 atoms, 120 ns (small: tables in full)
+    n, T, field = 5, 120, (0.3, 1.0, 0.5)
+    coords = W.disc_register(n, 30.0, 8.0, 9)
+    seq = Sequence(Register.from_coordinates(coords, center=False, prefix="q"), MockDevice)
+    seq.declare_channel("mw", "mw_global")
+    seq.set_magnetic_field(*field)
+    seq.add(Pulse.ConstantDetuning(BlackmanWaveform(T, 1.5 * np.pi), 0.8, 0), "mw")
+    put("xy", specs_of(seq)[0][0], tables=False)
+    np.savez_compressed(os.path.join(OUT, "pul_workloads.npz"), **out)
+    print("wrote pul_workloads")
+
+
+if __name__ == "__main__" and "--workloads" in sys.argv:
+    workloads()

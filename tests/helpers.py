@@ -1,6 +1,8 @@
 """Shared builders of seeded test inputs (no pulser needed)."""
 from __future__ import annotations
 
+import hashlib
+
 import numpy as np
 
 from pulser_b200 import workloads as W
@@ -48,3 +50,23 @@ def random_state(D: int, seed: int = 0) -> np.ndarray:
     rng = np.random.default_rng(seed)
     v = rng.normal(size=D) + 1j * rng.normal(size=D)
     return v / np.linalg.norm(v)
+
+
+def digest(a: np.ndarray) -> str:
+    """sha256 of an array's shape, dtype and values (-0.0 read as 0.0): equal digests mean equal arrays."""
+    a = np.ascontiguousarray(a) + np.zeros((), dtype=np.asarray(a).dtype)
+    return hashlib.sha256(f"{a.dtype.str}{a.shape}".encode() + a.tobytes()).hexdigest()
+
+
+def table_sample(a: np.ndarray, n: int = 64) -> tuple[np.ndarray, str]:
+    """A fixed, seeded sample of the columns (time samples) of a drive table, and the digest of the whole table."""
+    cols = np.sort(np.random.default_rng(0).choice(a.shape[-1], size=min(n, a.shape[-1]), replace=False))
+    return a[..., cols], digest(a)
+
+
+def assert_table_equal(a: np.ndarray, cols_ref: np.ndarray, digest_ref) -> None:
+    """``a`` equals the table that ``table_sample`` summarised: the sampled columns first (a readable failure), then
+    every element through the digest."""
+    cols, d = table_sample(a, cols_ref.shape[-1])
+    np.testing.assert_array_equal(cols, cols_ref)
+    assert d == str(digest_ref)

@@ -34,3 +34,37 @@ def test_reference_arm_line_contract():
 def test_reference_arm_other_ranks_stay_silent():
     res = _run({"RANK": "3", "WORLD_SIZE": "8"})
     assert res.returncode == 0 and res.stdout.strip() == ""
+
+
+def test_dump_outputs_format_and_sampling(tmp_path):
+    """bench.py --dump-outputs: the final state as float64 (re, im) pairs, the densities, and above the size cap a
+    seeded sample of amplitudes that is the same from run to run."""
+    code = (
+        "import sys, numpy as np; sys.path.insert(0, {root!r}); import bench\n"
+        "rng = np.random.default_rng(5); psi = rng.normal(size=64) + 1j * rng.normal(size=64)\n"
+        "bench.dump_outputs({full!r}, psi, np.arange(6.0))\n"
+        "bench.DUMP_BYTES = 16 * 16\n"
+        "bench.dump_outputs({a!r}, psi, np.arange(6.0)); bench.dump_outputs({b!r}, psi, np.arange(6.0))\n"
+    ).format(root=ROOT, full=str(tmp_path / "full"), a=str(tmp_path / "a"), b=str(tmp_path / "b"))
+    res = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300)
+    assert res.returncode == 0, res.stderr[-400:]
+    import numpy as np
+
+    rng = np.random.default_rng(5)
+    psi = rng.normal(size=64) + 1j * rng.normal(size=64)
+    full = np.load(tmp_path / "full" / "c2_state.npy")
+    assert full.dtype == np.float64 and full.shape == (64, 2)
+    np.testing.assert_array_equal(full[:, 0] + 1j * full[:, 1], psi)
+    assert sorted(os.listdir(tmp_path / "full")) == ["c2_rydberg_density.npy", "c2_state.npy"]
+    np.testing.assert_array_equal(np.load(tmp_path / "full" / "c2_rydberg_density.npy"), np.arange(6.0))
+    idx = np.load(tmp_path / "a" / "c2_state_index.npy")
+    part = np.load(tmp_path / "a" / "c2_state.npy")
+    assert idx.dtype == np.float64 and part.shape == (16, 2) and len(np.unique(idx)) == 16
+    np.testing.assert_array_equal(part, full[idx.astype(int)])
+    np.testing.assert_array_equal(idx, np.load(tmp_path / "b" / "c2_state_index.npy"))
+
+
+def test_steps_must_be_positive():
+    res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True,
+                         timeout=300)
+    assert res.returncode != 0 and "--steps" in res.stderr

@@ -3,8 +3,8 @@
 ``QutipBackendV2``, qutip_backend.py:235-325) driven by real ``pulser.Sequence`` objects through the real
 ``DevicePlan`` (no fake device), checked against the CPU oracle.
 
-pulser-core reaches the GPU box as the offline install under ``baseline/_ref`` (git-ignored, see DESIGN.md section 5);
-the tests skip where it is not importable.
+pulser-core reaches the GPU as the copy that build() makes under ``oracle/_ref`` (git-ignored, see DESIGN.md
+section 5); the tests skip where it is not importable.
 """
 from collections import Counter
 
